@@ -144,7 +144,7 @@ def run_reference(args, rank, world):
     cores = os.cpu_count()
     for i in range(min(args.warmup, 1)):
         cpu_reference_pair(frames[i % 2], cores)
-    steps = max(1, min(args.steps, 4))       # bounded sample: one frame pair (~5 s of CPU work) per step
+    steps = args.steps                       # one frame pair (~5 s of CPU work) per step
     t = [cpu_reference_pair(frames[i % 2], cores) for i in range(steps)]
     sec = sum(x[0] for x in t) / steps
     fps = 2.0 / sec
@@ -153,7 +153,7 @@ def run_reference(args, rank, world):
             "steps": steps, "warmup": min(args.warmup, 1), "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic", "impl": "reference",
             "config": {"workload": WORKLOAD, "maximum_features": MAXF, "detector_threshold": 0.001, "better_by": BETTER_BY, "arrsac": ARRSAC,
-                       "pairs_per_step": 1, "note": "bounded sample: one frame pair per step (the GPU arm's step is a batch of "
+                       "pairs_per_step": 1, "note": "one frame pair per step (the GPU arm's step is a batch of "
                                                     f"{PAIRS_PER_STEP} pairs); frames/s is step-size independent"},
             "cpu_baseline": {"value": fps, "unit": "frames/s", "cores": cores, "kind": "port",
                              "single_thread_value": 2.0 / sec1,
@@ -269,6 +269,38 @@ def track256(rank, world, ctxs):
             "timing": "host API (host pointers in, results on the host), wall clock, this rank's replica"}
 
 
+def dump_outputs(out_dir, pairs, pair_dev, slot, cap):
+    """--dump-outputs: what the device-resident path hands its caller for each frame pair of the last timed step, as .npy files
+    (float32 holds every index and keypoint field exactly; at most ~47 MB for 16 pairs of 5 000 keypoints per frame).  The pairs
+    run again, one at a time on context 0, after the timed region: a pair's result depends only on its frames and its generator
+    seed (the pair index), so it is the result the timed step computed.
+      keypoints   [N, 7]  x, y, response, size, angle, octave, class_id; frame a then frame b of each pair, in pair order
+      descriptors [N, 64] descriptor bytes, rows as in keypoints
+      matches     [M, 2]  keypoint index in frame a, keypoint index in frame b; in pair order
+      inliers     [I]     consensus inliers as indices into the pair's matches; in pair order
+      poses       [P, 12] consensus model (rotation row-major, translation); zero where none was found
+      counts      [P, 6]  pair index, keypoints in a, keypoints in b, matches, inliers, model found"""
+    from cv_b200._lib import KP_DTYPE
+    kps, descs, matches, inliers, poses, counts = [], [], [], [], [], []
+    for i in pairs:
+        pair_dev(i, 0)                  # returns with the context's stream drained
+        na, nb = slot.n.cpu().numpy().tolist()
+        npairs, ninl, found = slot.cnt.cpu().numpy()[:3].tolist()
+        kp = np.frombuffer(slot.kp.cpu().numpy().tobytes(), KP_DTYPE)
+        desc = slot.desc.cpu().numpy().reshape(2 * cap, 64)
+        for lo, n in ((0, na), (cap, nb)):
+            kps.append(np.stack([kp[f][lo:lo + n].astype(np.float32) for f in KP_DTYPE.names], 1))
+            descs.append(desc[lo:lo + n].astype(np.float32))
+        matches.append(slot.pairs.cpu().numpy()[:2 * npairs].reshape(-1, 2).astype(np.float32))
+        inliers.append(slot.inl.cpu().numpy()[:ninl].astype(np.float32))
+        poses.append(slot.model.cpu().numpy() if found else np.zeros(12))
+        counts.append([i, na, nb, npairs, ninl, found])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("keypoints", np.concatenate(kps)), ("descriptors", np.concatenate(descs)), ("matches", np.concatenate(matches)),
+                    ("inliers", np.concatenate(inliers)), ("poses", np.stack(poses)), ("counts", np.array(counts, np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def bind_to_gpu_numa_node(props):
     """Run this process (and the pinned buffers it first-touches) on the CPUs local to the GPU's PCIe root, like a deployed
     service would; silently skipped when sysfs does not expose the topology."""
@@ -292,7 +324,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="cvb200")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step's frame pairs to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path only")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -313,7 +351,7 @@ def main():
     dev = torch.device("cuda", local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    K, Wm = max(args.steps, 1), max(args.warmup, 3)          # timing rule: at least 3 warm-up steps
+    K, Wm = args.steps, max(args.warmup, 3)          # timing rule: at least 3 warm-up steps
     NCTX = int(os.environ.get("CVB_BENCH_CONTEXTS", "16"))   # 16 contexts x (main + auxiliary stream) = the 32 hardware queues: more contexts alias queues   # contexts (stream + workspace + host thread each) pipelined on the GPU
 
     frames = make_pool(POOL_PAIRS, seed0=100 * rank)
@@ -333,8 +371,8 @@ def main():
     h_pool = [torch.from_numpy(p).pin_memory() for p in frames]
 
     class Slot:
-        """Everything one context owns: device result buffers, pinned host result buffers, its consensus generator (the
-        two_view_consensus object of a VSlam instance keeps its generator across frame pairs)."""
+        """Everything one context owns: device result buffers, pinned host result buffers, its consensus generator (pair_dev
+        seeds it per pair; pair_host carries it across frame pairs, like the two_view_consensus object of a VSlam instance)."""
         def __init__(self):
             self.kp = torch.empty(2 * cap * KP_DTYPE.itemsize, dtype=torch.uint8, device=dev)
             self.desc = torch.zeros(2 * cap * 64, dtype=torch.uint8, device=dev)
@@ -358,9 +396,11 @@ def main():
     slots = [Slot() for _ in range(NCTX)]
 
     def pair_dev(i, c):
-        """device-resident: frames already in HBM, results stay in HBM; one synchronisation (the generator commit)"""
+        """device-resident: frames already in HBM, results stay in HBM; one synchronisation (the generator commit).  The
+        consensus generator is seeded with the pair index, so pair i's result does not depend on which context ran it."""
         cx, s = ctxs[c], slots[c]
         img = d_pool[i % POOL_PAIRS]
+        lib.cvb_rng_seed_xoshiro256pp(C.byref(s.rng), i)
         cx.check(lib.cvb_akaze_extract_batch_dev(cx.handle, C.byref(akaze_cfg), img.data_ptr(), 2, W, H, s.kp.data_ptr(), s.desc.data_ptr(), cap,
                                                  s.n.data_ptr()))
         cx.check(lib.cvb_two_view_pair_dev(cx.handle, s.kp.data_ptr(), s.desc.data_ptr(), s.n.data_ptr(),
@@ -445,6 +485,8 @@ def main():
     stats0 = [int(x) for x in slots[0].stats]
     n_kp = slots[0].n.cpu().numpy().tolist()
     cnt0 = slots[0].cnt.cpu().numpy().tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, range((Wm + K - 1) * PAIRS_PER_STEP, (Wm + K) * PAIRS_PER_STEP), pair_dev, slots[0], cap)
 
     # ---- e2e: host entry point, pinned host buffers, copies inside the timed region
     reset_rngs()
@@ -538,7 +580,6 @@ def main():
     # ---- roofline: instrumented pass (per-kernel CUDA events on the launching stream, one context, no overlap)
     ctx.profile(True)
     PK = 6
-    lib.cvb_rng_seed_xoshiro256pp(C.byref(slots[0].rng), 0)
     for i in range(PK):
         pair_dev(i, 0)
     rep = ctx.profile_report()

@@ -1,5 +1,5 @@
 import sys, os, time
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..', '..'))
 import numpy as np
 from oracle import pyoracle as O
 from tests.synth import synth_frame, warp_frame

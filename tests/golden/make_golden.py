@@ -1,8 +1,11 @@
-"""Generates the golden fixtures under tests/golden/ (run in the build container, where
-/root/reference exists; the GPU box never reads /root/reference).
+"""Generates the golden fixtures under tests/golden/ from a checkout of the reference (rust-cv/cv):
+
+    python tests/golden/make_golden.py <reference checkout>
+
+The tests read only the stored fixtures, never the reference checkout.
 
  - kitti_0000000000.npz / kitti_0000000014.npz : the two reference fixture frames
-   (/root/reference/res/*.png, 1392x512 8-bit gray) as uint8 arrays -- inputs of the reference's
+   (res/*.png of the reference, 1392x512 8-bit gray) as uint8 arrays -- inputs of the reference's
    own golden test akaze/tests/estimate_pose.rs:24-76.
  - akaze_goldens.json : the counts that test asserts (399 / 343 descriptors, 11 Lowe-0.5 matches,
    estimate_pose.rs:41-42,59) plus secondary counts produced by the oracle at Akaze::default().
@@ -20,13 +23,11 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 from oracle import pyoracle as O  # noqa: E402
 
-REF = "/root/reference/res"
 
-
-def main():
+def main(ref_root):
     frames = {}
     for name in ("0000000000", "0000000014"):
-        im = cv2.imread(os.path.join(REF, name + ".png"), cv2.IMREAD_UNCHANGED)
+        im = cv2.imread(os.path.join(ref_root, "res", name + ".png"), cv2.IMREAD_UNCHANGED)
         assert im.dtype == np.uint8 and im.ndim == 2
         np.savez_compressed(os.path.join(HERE, f"kitti_{name}.npz"), image=im)
         frames[name] = im.astype(np.float32) / np.float32(255)  # GrayFloatImage::from_dynamic, image.rs:53-55
@@ -56,4 +57,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])
